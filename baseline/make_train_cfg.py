@@ -1,6 +1,7 @@
 """Dumps the widowGo1 training configuration of the reference (WidowGo1RoughCfgPPO, legged_gym/envs/widowGo1/widowGo1_config.py:317-383)
-to baseline/widowgo1_train_cfg.json, so that bench.py can construct the reference's own ActorCritic / PPO on the GPU box, where
-legged_gym (which needs isaacgym) is absent.  Run in the authoring container:  python baseline/make_train_cfg.py"""
+to baseline/widowgo1_train_cfg.json, so that bench.py can construct the reference's own ActorCritic / PPO where
+legged_gym (which needs isaacgym) cannot be imported.  Run with a checkout of the original repository:
+DWBC_REFERENCE=<checkout> python baseline/make_train_cfg.py"""
 import json
 import os
 import sys

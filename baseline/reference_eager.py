@@ -20,7 +20,7 @@ REF = os.path.join(HERE, "_ref")
 def available() -> str | None:
     """None if the reference install is usable, else a one-line reason."""
     if not os.path.isdir(os.path.join(REF, "rsl_rl")):
-        return "baseline/_ref/rsl_rl is absent (run baseline/install_reference.sh in the authoring container)"
+        return "baseline/_ref/rsl_rl is absent (run baseline/install_reference.sh with DWBC_REFERENCE set to a checkout of the original project)"
     return None
 
 

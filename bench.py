@@ -11,6 +11,7 @@ One "step" = one PPO iteration over one batch of synthetic sim-state tensors:
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (configs[1]: flat terrain, 4096 envs/GPU)
     python bench.py --config rough | roa                             # configs[2] (height scan + terrain curriculum) / configs[3] (ROA, 8192 envs)
     python bench.py --impl reference [--gpus N] --steps K --warmup W   # the reference path on host cores, same config
+    python bench.py --steps K --warmup W --dump-outputs DIR          # + what the last timed step computed, as DIR/*.npy
 
 The headline runs the error-compensated tensor-core path (`--precision tf32x3`: fp32-grade, passes the fp32 parity assertions of
 tests/test_gpu_ppo.py); the line also carries the plain-TF32 numbers (`tf32`) and, report-only, the reference's own rsl_rl as eager
@@ -223,6 +224,35 @@ class Workload:
         self.obs = obs
 
 
+DUMP_LIMIT_BYTES = 64 * 2**20
+DUMP_ENVS = 4096            # per-env arrays of a larger run (roa: 8192 envs) are a fixed, seeded sample of this many envs
+DUMP_OBS_ROWS = 2048        # rollout observations [T, N, 860] (563 MB at 4096 envs): a fixed, seeded sample of (t, env) rows
+
+
+def dump_outputs(w, out_dir):
+    """Writes what the last timed iteration handed its caller as out_dir/<name>.npy: update()'s losses, the parameters after the
+    update, the rollout storage it trained on and the last observation.  The samples are drawn from a fixed seed, so two runs
+    with the same arguments write the same rows.  The weight gradients are summed with float atomics in no fixed order, so the
+    parameters, and everything computed from them in later iterations, agree between two runs to rounding, not bit for bit."""
+    s, N, T = w.alg.storage, w.N, w.T
+    g = torch.Generator().manual_seed(0)
+    envs = torch.arange(N) if N <= DUMP_ENVS else torch.randperm(N, generator=g)[:DUMP_ENVS].sort().values
+    rows = torch.randperm(T * N, generator=g)[:DUMP_OBS_ROWS].sort().values
+    envs, rows = envs.to(w.device), rows.to(w.device)
+    out = {"update_losses": torch.tensor(w.last, dtype=torch.float64),
+           "params": torch.cat([v.reshape(-1) for v in w.alg.actor_critic.state_dict().values()]),
+           "last_obs": w.obs[envs],
+           "observations_sample": s.observations.reshape(T * N, -1)[rows]}
+    for k in ("actions", "actions_log_prob", "values", "rewards", "dones", "returns", "advantages"):
+        out[k] = getattr(s, k)[:, envs]
+    out = {k: (v.cpu().numpy() if v.dtype == torch.float64 else v.float().cpu().numpy()) for k, v in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_LIMIT_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def cuda_ms(fn, reps, barrier, device, world):
     """fn() `reps` times between CUDA events, max over ranks."""
     import torch.distributed as dist
@@ -294,6 +324,8 @@ def run_ours(args):
         sampler.start()
     ms, launches = timed(w, args.steps, time_k1=True)
     clocks = sampler.finish() if sampler else None
+    if args.dump_outputs and rank == 0:       # before the measurements below move the workload on
+        dump_outputs(w, args.dump_outputs)
     k1_ms = float(np.mean([a.elapsed_time(b) for a, b in w.k1_events])) if w.k1_events else None
     value = world * w.N * w.T * args.steps / (ms / 1e3)
 
@@ -455,8 +487,8 @@ def mlp_roofline(update_ms, mb_rows, pk, precision):
 # ------------------------------------------------------------------------------------------------
 # CPU legs: the reference's algorithm on the box's host cores, at the metric's own config (4096 envs x 40 steps).
 # Update half = the UNMODIFIED reference rsl_rl (baseline/_ref: PPO.act / process_env_step / compute_returns / update) when it
-# travelled with the snapshot; env half = the oracle port of WidowGo1.post_physics_step (the reference env imports the closed
-# isaacgym package and /root/reference does not exist on the GPU box).
+# is installed (baseline/install_reference.sh), else the oracle port; env half = the oracle port of WidowGo1.post_physics_step (the
+# reference env imports the closed isaacgym package).
 # ------------------------------------------------------------------------------------------------
 def make_oracle_iteration(n_envs, T, seed=100):
     import envstate as E
@@ -513,7 +545,7 @@ class CpuIteration:
 
 def pick_threads(n_envs=256):
     """torch CPU intra-op threading is counter-productive past a point for these op sizes (128
-    OpenMP threads were 30x SLOWER than 8 on the GPU box's host): probe a short slice of the
+    OpenMP threads were 30x SLOWER than 8 on a 128-core host): probe a short slice of the
     workload at several thread counts up to all cores and keep the fastest, i.e. give the CPU arm
     its best configuration.  Returns (threads_used, host_cores)."""
     cores = os.cpu_count() or 1
@@ -554,7 +586,7 @@ def run_reference(args):
     n_envs = N_ENVS
     cores, host_cores = pick_threads(512)
     it = CpuIteration(n_envs, T_STEPS)
-    steps, warmup = max(1, min(args.steps, 12)), min(args.warmup, 1)      # ~5 s per iteration: bounded so that the run ends within minutes
+    steps, warmup = args.steps, min(args.warmup, 1)      # ~5 s per iteration: one warm-up iteration is enough on the host
     for _ in range(warmup):
         it.run()
     t0 = time.perf_counter()
@@ -563,7 +595,7 @@ def run_reference(args):
     dt = time.perf_counter() - t0
     value = n_envs * T_STEPS * steps / dt
     sample = (f"each step = one full PPO iteration at the metric's config ({n_envs} envs x {T_STEPS} steps) on {cores} torch threads "
-              f"(fastest of a probe up to all {host_cores} host cores); {steps} timed steps (of the {args.steps} asked for: bounded to a few minutes)")
+              f"(fastest of a probe up to all {host_cores} host cores); {steps} timed steps")
     print(json.dumps({
         "impl": "reference", "metric": "env-steps/sec (widowGo1, 4096 envs/GPU)", "value": value, "unit": "env-steps/s",
         "n_gpus": int(os.environ.get("WORLD_SIZE", 1)), "steps": steps, "warmup": warmup, "ms_per_step": dt / steps * 1e3,
@@ -585,7 +617,14 @@ if __name__ == "__main__":
     ap.add_argument("--precision", default="tf32x3", choices=["fp32", "tf32", "tf32x3"],
                     help="ActorCritic GEMM arithmetic: tf32x3 = error-compensated tensor cores (default: fp32-grade, passes the fp32 parity tests), "
                          "tf32 = plain TF32 tensor cores (what the reference's pinned torch 1.10 does on Ampere+, allow_tf32=True), fp32 = CUDA cores")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (losses, parameters, rollout storage, last observation; "
+                         "rank 0) as DIR/<name>.npy, at most 64 MB")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if a.impl == "reference":
         run_reference(a)
     else:

@@ -1,11 +1,11 @@
 """Generate the golden vectors under tests/golden/ by EXECUTING THE UNMODIFIED REFERENCE.
 
-Run in the authoring container only (needs /root/reference):
+Needs a checkout of the original Deep-Whole-Body-Control repository, named by DWBC_REFERENCE:
 
-    python tests/golden/make_golden.py
+    DWBC_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 For each fixture the script (1) runs the reference's own Python on CPU (env half through the
-fake isaacgym of tests/fakes, update half straight from /root/reference/rsl_rl), (2) runs the
+fake isaacgym of tests/fakes, update half straight from its rsl_rl), (2) runs the
 restatement in oracle/ on the same inputs and ASSERTS it reproduces the reference (this is
 what pins the oracle), (3) stores the reference outputs.  Inputs are not stored: they are
 regenerated from (seed, stream) by dwbc_b200.synth (integer-hash, machine independent).

@@ -1,6 +1,6 @@
 """Golden vectors of `WidowGo1._compute_torques` (WG:1262-1295): the UNMODIFIED reference method is called on a stub object
 holding exactly the attributes it reads; asserts oracle == reference and writes tests/golden/torques.npz.
-Run in the authoring container only:  python tests/golden/make_golden_torques.py"""
+Run with a checkout of the original repository:  DWBC_REFERENCE=<checkout> python tests/golden/make_golden_torques.py"""
 import os
 import sys
 from types import SimpleNamespace

@@ -1,7 +1,8 @@
-"""Executes the UNMODIFIED reference (`/root/reference`) on CPU for golden-vector generation.
+"""Executes the UNMODIFIED reference on CPU for golden-vector generation: the checkout of the original
+Deep-Whole-Body-Control repository (legged_gym/, rsl_rl/) that the environment variable DWBC_REFERENCE names.
 
-Runs only in the authoring container (the GPU box has no /root/reference).  Nothing here is
-imported by the test-suite proper; tests read the .npz files this produces.
+The tests proper read the .npz files this produces; only the check of the default parameters against the
+reference config (tests/test_host_cpu.py) imports it, and it skips without DWBC_REFERENCE.
 
 Recipe = SURVEY.md Appendix A: fake `isaacgym` (tests/fakes), `WidowGo1.__new__`, synthetic
 state tensors, then the reference's own `post_physics_step()`.  The reference draws randoms
@@ -21,7 +22,9 @@ import numpy as np
 import torch
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), "..", ".."))
-REF = "/root/reference"
+REF = os.environ.get("DWBC_REFERENCE", "")
+if not (REF and os.path.isdir(os.path.join(REF, "legged_gym"))):
+    raise ImportError("set DWBC_REFERENCE to a checkout of the original Deep-Whole-Body-Control repository (legged_gym/, rsl_rl/)")
 for pth in (ROOT, os.path.join(ROOT, "tests", "fakes"), os.path.join(REF, "legged_gym"), os.path.join(REF, "rsl_rl")):
     if pth not in sys.path:
         sys.path.insert(0, pth)

@@ -61,7 +61,7 @@ class SyntheticWidowGo1(object):
         return self.core.step(actions, physics=self._physics)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "rsl_rl")), reason="baseline/_ref (unmodified rsl_rl) is absent")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "rsl_rl")), reason="baseline/_ref (unmodified rsl_rl) is absent: run baseline/install_reference.sh")
 def test_unmodified_on_policy_runner_drives_the_fused_classes(tmp_path):
     import json
     for pth in (REF, os.path.join(ROOT, "tests", "fakes")):

@@ -223,7 +223,8 @@ def test_storage_shapes_follow_reference():
     assert len(batches) == 12 and all(b.numel() == 10 for b in batches) and torch.equal(batches[0], batches[4])     # RS:182-188 order
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/legged_gym"), reason="authoring container only: needs the reference's config module")
+@pytest.mark.skipif(not (os.environ.get("DWBC_REFERENCE") and os.path.isdir(os.path.join(os.environ["DWBC_REFERENCE"], "legged_gym"))),
+                    reason="needs the original project's legged_gym config module: set DWBC_REFERENCE to a checkout of it")
 def test_default_params_equal_the_reference_config():
     """`WidowGo1Params()` hard-codes the widowGo1 constants so that the kernels can run without legged_gym; this pins every one of them
     (dims, ranges, thresholds, curricula, PD gains, action scale, active reward terms and scales) to `WidowGo1RoughCfg` as shipped, read
