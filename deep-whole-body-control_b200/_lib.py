@@ -12,7 +12,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libdwbc.so")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_DOF, MAX_TERMS, MAX_IDX, MAX_SLOTS, NUM_METRICS, RAND_COLS, MAX_LAYERS = 24, 40, 8, 64, 10, 104, 4
 GS, DS = 28, 72
 GS_COL = dict(commands=0, goal_timer=3, traj_timesteps=4, traj_total_timesteps=5, ee_start_sphere=6, ee_goal_sphere=9,
@@ -93,11 +93,13 @@ class NetCfg(C.Structure):
         ("off_critic_w", i64 * MAX_LAYERS), ("off_critic_b", i64 * MAX_LAYERS),
         ("off_cleg_w", i64 * (MAX_LAYERS + 1)), ("off_cleg_b", i64 * (MAX_LAYERS + 1)),
         ("off_carm_w", i64 * (MAX_LAYERS + 1)), ("off_carm_b", i64 * (MAX_LAYERS + 1)),
-        ("precision", i32), ("reserved_", i32),
+        ("precision", i32), ("activation", i32),
     ]
 
 
 PRECISIONS = {"fp32": 0, "tf32": 1, "tf32x3": 2}
+# rsl_rl `get_activation` names (AC) -> DwbcActivation; "crelu" is rsl_rl's name for a plain nn.ReLU()
+ACTIVATIONS = {"elu": 0, "selu": 1, "relu": 2, "crelu": 2, "lrelu": 3, "tanh": 4, "sigmoid": 5}
 
 
 class PpoHyper(C.Structure):

@@ -63,8 +63,9 @@ class FlatActorCritic:
 
     def __init__(self, num_actor_obs=76, num_critic_obs=76, num_actions=18, actor_hidden_dims=(128,), critic_hidden_dims=(128,),
                  priv_encoder_dims=(64, 20), activation="elu", init_std=None, device="cuda:0", seed=None, **kwargs):
-        if activation != "elu":
-            raise L.DwbcError("only activation='elu' (WGC:325) is implemented by the kernels")
+        if activation not in L.ACTIVATIONS:
+            raise L.DwbcError(f"activation={activation!r}: rsl_rl's get_activation offers {sorted(L.ACTIVATIONS)}")
+        self.activation = activation
         if kwargs.get("adaptive_arm_gains", False):
             raise L.DwbcError("adaptive_arm_gains=True is outside the hot path (WGC:168: False)")
         self.num_prop = kwargs.get("num_prop", num_actor_obs)
@@ -123,6 +124,7 @@ class FlatActorCritic:
         dims("n_arm_layers", "arm_dims", self.arm_dims)
         c.hist_proj, c.hist_c1, c.hist_k1, c.hist_s1, c.hist_c2, c.hist_k2, c.hist_s2 = 30, 20, 4, 2, 10, 2, 1
         c.num_params, c.off_std = self.num_params, o["std"]
+        c.activation = L.ACTIVATIONS[self.activation]
 
         def offs(w_attr, b_attr, prefix, n):
             for i in range(n):

@@ -14,7 +14,22 @@
 
 namespace dwbc {
 
-enum { ACT_NONE = 0, ACT_ELU = 1, ACT_TANH = 2 };
+// activation codes of the layer ops (GemmArgs.act, C2Op.act): the heads' outputs use NONE / TANH, every hidden layer the network's
+// DwbcNetCfg.activation (act_code)
+enum { ACT_NONE = 0, ACT_ELU = 1, ACT_TANH = 2, ACT_SELU = 3, ACT_RELU = 4, ACT_LRELU = 5, ACT_SIGMOID = 6, ACT_COUNT = 7 };
+constexpr float SELU_SCALE = 1.0507009873554805f, SELU_ALPHA = 1.6732632423543772f, LRELU_SLOPE = 0.01f;
+// DwbcActivation (ABI) -> activation code; -1: unknown
+inline int act_code(int32_t abi_act) {
+  switch (abi_act) {
+    case DWBC_ACT_ELU: return ACT_ELU;
+    case DWBC_ACT_SELU: return ACT_SELU;
+    case DWBC_ACT_RELU: return ACT_RELU;
+    case DWBC_ACT_LRELU: return ACT_LRELU;
+    case DWBC_ACT_TANH: return ACT_TANH;
+    case DWBC_ACT_SIGMOID: return ACT_SIGMOID;
+    default: return -1;
+  }
+}
 
 struct RowMat {
   const float* p;       // base (already offset to the first column)
@@ -41,6 +56,29 @@ inline RowMat rowmat_grouped(const float* p, const int64_t* idx, int rpg, int64_
 }
 
 __device__ __forceinline__ float elu_f(float x) { return x > 0.0f ? x : expf(x) - 1.0f; }
+// exact fp32 forms (precise expf / tanhf) of every activation, the derivative written in terms of the OUTPUT y = f(x)
+__device__ __forceinline__ float act_f(int act, float x) {
+  switch (act) {
+    case ACT_ELU: return elu_f(x);
+    case ACT_TANH: return tanhf(x);
+    case ACT_SELU: return x > 0.0f ? SELU_SCALE * x : (SELU_SCALE * SELU_ALPHA) * (expf(x) - 1.0f);
+    case ACT_RELU: return fmaxf(x, 0.0f);
+    case ACT_LRELU: return x > 0.0f ? x : x * LRELU_SLOPE;
+    case ACT_SIGMOID: return 1.0f / (1.0f + expf(-x));
+    default: return x;
+  }
+}
+__device__ __forceinline__ float act_dy(int act, float y) {
+  switch (act) {
+    case ACT_ELU: return y > 0.0f ? 1.0f : y + 1.0f;
+    case ACT_TANH: return 1.0f - y * y;
+    case ACT_SELU: return y > 0.0f ? SELU_SCALE : y + SELU_SCALE * SELU_ALPHA;
+    case ACT_RELU: return y > 0.0f ? 1.0f : 0.0f;
+    case ACT_LRELU: return y > 0.0f ? 1.0f : LRELU_SLOPE;
+    case ACT_SIGMOID: return y * (1.0f - y);
+    default: return 1.0f;
+  }
+}
 
 constexpr int GT_M = 64, GT_N = 64, GT_K = 16, GT_PAD = 4, GT_THREADS = 256;
 
@@ -190,10 +228,12 @@ __global__ void __launch_bounds__(GT_THREADS) gemm_tile_kernel(const GemmArgs g)
         if (g.bias) v += g.bias[n];
         if (g.act == ACT_ELU) v = elu_f(v);
         else if (g.act == ACT_TANH) v = tanhf(v);
+        else if (g.act != ACT_NONE) v = act_f(g.act, v);
       } else if (xrow) {
         const float y = xrow[n];
         if (g.act == ACT_ELU) v *= (y > 0.0f ? 1.0f : y + 1.0f);
         else if (g.act == ACT_TANH) v *= (1.0f - y * y);
+        else v *= act_dy(g.act, y);
       }
       crow[n] = v;
     }

@@ -28,6 +28,16 @@ __device__ __forceinline__ void t2_arrive(uint64_t* bar) {
 // tanh for the TF32 path: 1 - 2/(e^{2x}+1) with ex2.approx / rcp.approx (a few ulp; saturates correctly at +-inf). Short enough that an
 // if-converted activation select costs nothing for the ELU layers (precise tanhf is ~60 predicated instructions per element).
 __device__ __forceinline__ float t2_tanh(float x) { return 1.0f - __fdividef(2.0f, __expf(2.0f * x) + 1.0f); }
+// the other hidden activations on the TF32 paths (ex2.approx / rcp.approx like t2_tanh; ELU and tanh keep their own lines)
+__device__ __forceinline__ float t2_act(int act, float x) {
+  switch (act) {
+    case ACT_SELU: return x > 0.0f ? SELU_SCALE * x : (SELU_SCALE * SELU_ALPHA) * (__expf(x) - 1.0f);
+    case ACT_RELU: return fmaxf(x, 0.0f);
+    case ACT_LRELU: return x > 0.0f ? x : x * LRELU_SLOPE;
+    case ACT_SIGMOID: return __fdividef(1.0f, 1.0f + __expf(-x));
+    default: return act_f(act, x);
+  }
+}
 // named barriers are the warp-aligned form: reconverge the warp first (a lane may still be behind a single-lane mbarrier arrive)
 __device__ __forceinline__ void t2_pbar() { __syncwarp(); asm volatile("bar.sync 2, %0;" ::"n"(T2_PROD) : "memory"); }   // producers only
 __device__ __forceinline__ void t2_ebar() { __syncwarp(); asm volatile("bar.sync 3, %0;" ::"n"(T2_EPI) : "memory"); }    // epilogue only
@@ -284,8 +294,10 @@ __global__ void __launch_bounds__(T2_THREADS, 1) gemm_tc2_kernel(const GemmArgs 
                   if (vecB & 8) { }
                   else if (g.act == ACT_ELU) tt = tt > 0.0f ? tt : __expf(tt) - 1.0f;   // ex2.approx: 2 ulp, far below the TF32 input rounding
                   else if (g.act == ACT_TANH) tt = t2_tanh(tt);
+                  else if (g.act != ACT_NONE) tt = t2_act(g.act, tt);
                 } else if (g.act == ACT_ELU) tt *= (y[u][qq] > 0.0f ? 1.0f : y[u][qq] + 1.0f);
                 else if (g.act == ACT_TANH) tt *= (1.0f - y[u][qq] * y[u][qq]);
+                else if (g.act != ACT_NONE) tt *= act_dy(g.act, y[u][qq]);
                 x[u][qq] = tt;
               }
             }

@@ -1,5 +1,5 @@
-// History encoder (StateHistoryEncoder, AC:39-84: Linear 76->30 + ELU per time step, Conv1d(30->20, k=4, s=2) + ELU, Conv1d(20->10, k=2, s=1) + ELU,
-// Flatten, Linear 30->latent + ELU) as ONE exact-fp32 kernel for the inference uses: the regulariser target of PPO.update (PPO:175-176, no
+// History encoder (StateHistoryEncoder, AC:39-84: Linear 76->30 + act per time step, Conv1d(30->20, k=4, s=2) + act, Conv1d(20->10, k=2, s=1) + act,
+// Flatten, Linear 30->latent + act; act = the network's hidden activation, ELU in the shipped config) as ONE exact-fp32 kernel for the inference uses: the regulariser target of PPO.update (PPO:175-176, no
 // gradient), rollouts with hist_encoding (AC:207-210) and act_inference.  The layer-wise path needs four GEMM launches plus packing / padding
 // kernels and moves the [rows x 10 x 32] projection through HBM; here a thread owns a row, streams its 10 x 76 history once (the only HBM
 // traffic: 3 040 B per row), and keeps every intermediate in registers:
@@ -28,8 +28,12 @@ struct HistFusedArgs {
   int rows, latent;
 };
 
-__device__ __forceinline__ float hf_elu(float x) { return x > 0.0f ? x : expf(x) - 1.0f; }     // precise expf: this is the exact path
+// the hidden activation, precise expf / tanhf: this is the exact path.  One kernel per activation (kAct is a compile-time constant,
+// so the ELU instance is the plain ELU line)
+template <int kAct>
+__device__ __forceinline__ float hf_act(float x) { return kAct == ACT_ELU ? (x > 0.0f ? x : expf(x) - 1.0f) : act_f(kAct, x); }
 
+template <int kAct>
 __global__ void __launch_bounds__(HF_THREADS) hist_fused_kernel(const HistFusedArgs a) {
   __shared__ __align__(16) float w[HF_FLOATS];
   // ---- weights -> shared memory, transposed to [input][output] (pads zero) ----
@@ -57,7 +61,7 @@ __global__ void __launch_bounds__(HF_THREADS) hist_fused_kernel(const HistFusedA
   float4 xnext = __ldg(reinterpret_cast<const float4*>(hp));
 #pragma unroll 1
   for (int t = 0; t < 10; ++t) {
-    // ---- projection of step t: h = ELU(Wp x + bp) ----
+    // ---- projection of step t: h = act(Wp x + bp) ----
     float h[32];
 #pragma unroll
     for (int o = 0; o < 32; ++o) h[o] = w[HF_BP + o];
@@ -81,7 +85,7 @@ __global__ void __launch_bounds__(HF_THREADS) hist_fused_kernel(const HistFusedA
       }
     }
 #pragma unroll
-    for (int o = 0; o < 30; ++o) h[o] = hf_elu(h[o]);
+    for (int o = 0; o < 30; ++o) h[o] = hf_act<kAct>(h[o]);
     // ---- conv 1: step t is tap (t & 1) + 2 of position p - 1 and tap t & 1 of position p = t / 2 ----
     const int kb = t & 1, ka = kb + 2;
     if (t >= 2) {
@@ -115,7 +119,7 @@ __global__ void __launch_bounds__(HF_THREADS) hist_fused_kernel(const HistFusedA
         // position q = (t - 3) / 2 of conv 1 is complete
         const int q = (t - 3) >> 1;
 #pragma unroll
-        for (int o = 0; o < 20; ++o) c1a[o] = hf_elu(c1a[o]);
+        for (int o = 0; o < 20; ++o) c1a[o] = hf_act<kAct>(c1a[o]);
         if (q >= 1) {
           // conv 2 position q - 1 = taps (c1[q-1], c1[q]); then its share of the output layer
           float c2[12];
@@ -135,7 +139,7 @@ __global__ void __launch_bounds__(HF_THREADS) hist_fused_kernel(const HistFusedA
           const float* wl = w + HF_WL + (q - 1) * 10 * 32;
 #pragma unroll
           for (int c = 0; c < 10; ++c) {
-            const float cv = hf_elu(c2[c]);
+            const float cv = hf_act<kAct>(c2[c]);
             const float4* wr = reinterpret_cast<const float4*>(wl + c * 32);
 #pragma unroll
             for (int o4 = 0; o4 < 8; ++o4) {
@@ -155,13 +159,22 @@ __global__ void __launch_bounds__(HF_THREADS) hist_fused_kernel(const HistFusedA
   float* orow = a.out + (int64_t)r * a.ld_out;
 #pragma unroll
   for (int o = 0; o < 32; ++o)
-    if (o < a.ld_out) orow[o] = o < a.latent ? hf_elu(z[o]) : 0.0f;
+    if (o < a.ld_out) orow[o] = o < a.latent ? hf_act<kAct>(z[o]) : 0.0f;
 }
 
 // latent <= 32, ld_out <= 32, history rows 16-byte aligned
-inline int launch_hist_fused(const HistFusedArgs& a, cudaStream_t st) {
+inline int launch_hist_fused(const HistFusedArgs& a, int act, cudaStream_t st) {
   if (a.rows <= 0 || a.latent > 32 || a.ld_out > 32 || a.ld_out < a.latent) return DWBC_ERR_UNSUPPORTED;
-  hist_fused_kernel<<<(a.rows + HF_THREADS - 1) / HF_THREADS, HF_THREADS, 0, st>>>(a);
+  const unsigned grid = (a.rows + HF_THREADS - 1) / HF_THREADS;
+  switch (act) {
+    case ACT_ELU: hist_fused_kernel<ACT_ELU><<<grid, HF_THREADS, 0, st>>>(a); break;
+    case ACT_SELU: hist_fused_kernel<ACT_SELU><<<grid, HF_THREADS, 0, st>>>(a); break;
+    case ACT_RELU: hist_fused_kernel<ACT_RELU><<<grid, HF_THREADS, 0, st>>>(a); break;
+    case ACT_LRELU: hist_fused_kernel<ACT_LRELU><<<grid, HF_THREADS, 0, st>>>(a); break;
+    case ACT_TANH: hist_fused_kernel<ACT_TANH><<<grid, HF_THREADS, 0, st>>>(a); break;
+    case ACT_SIGMOID: hist_fused_kernel<ACT_SIGMOID><<<grid, HF_THREADS, 0, st>>>(a); break;
+    default: return DWBC_ERR_ARG;
+  }
   ++dwbc_launch_counter;
   return cudaGetLastError() == cudaSuccess ? DWBC_OK : DWBC_ERR_LAUNCH;
 }

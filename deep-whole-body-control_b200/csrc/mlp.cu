@@ -1,6 +1,6 @@
 // ActorCritic forward / PPO loss / hand-written backward, fp32 CUDA-core path (K5-K8 anchor).
 //
-// Layer-wise: every nn.Linear (+ELU/Tanh) of `rsl_rl/modules/actor_critic.py` is one launch of
+// Layer-wise: every nn.Linear (+activation) of `rsl_rl/modules/actor_critic.py` is one launch of
 // the tile GEMM in gemm_simt.cuh with the bias/activation (forward) or activation derivative
 // (backward) fused into its epilogue; the mini-batch gather (RS:189-201) is fused into the
 // first-layer operand loads (no gathered batch is materialised); the Conv1d history encoder
@@ -125,7 +125,7 @@ static Plan make_plan(const DwbcNetCfg& n, int64_t rows, void* ws) {
 }
 
 static int check_net(const DwbcNetCfg* n) {
-  if (!n || n->abi_version != DWBC_ABI_VERSION || n->precision < 0 || n->precision > 2) return DWBC_ERR_ARG;
+  if (!n || n->abi_version != DWBC_ABI_VERSION || n->precision < 0 || n->precision > 2 || act_code(n->activation) < 0) return DWBC_ERR_ARG;
   mlp_precision = n->precision;
   if (n->n_priv_layers < 1 || n->n_priv_layers > DWBC_MAX_LAYERS || n->n_actor_layers < 1 || n->n_actor_layers > DWBC_MAX_LAYERS ||
       n->n_critic_layers < 1 || n->n_critic_layers > DWBC_MAX_LAYERS || n->n_leg_layers < 1 || n->n_leg_layers > DWBC_MAX_LAYERS ||
@@ -138,6 +138,9 @@ static int check_net(const DwbcNetCfg* n) {
   if (last(n->priv_dims, n->n_priv_layers) > 32 || n->n_leg + n->n_arm > 32) return DWBC_ERR_UNSUPPORTED;
   return DWBC_OK;
 }
+
+// activation code of every hidden layer (check_net has validated it)
+static inline int hid(const DwbcNetCfg& n) { return act_code(n.activation); }
 
 // ---- history-encoder weight re-packing ---------------------------------------------------------
 // conv1 [20,30,4] -> W1'[20][k*32+cin]; conv2 [10,20,2] -> W2'[10][k*20+cin]; linear [L,30] over the
@@ -175,10 +178,10 @@ __global__ void hist_unpack_grad_kernel(const float* __restrict__ g1, const floa
     if (c2 < 10) wl[j * 30 + c2 * 3 + t] = gl[i];
   }
 }
-// col2im of the conv input gradients (overlapping windows) fused with the ELU derivative:
-// dst[m][t][c] = elu'(y[m][t][c]) * sum_{t'*stride + k == t} src[(m*To + t')][k*C + c]
+// col2im of the conv input gradients (overlapping windows) fused with the activation derivative:
+// dst[m][t][c] = act'(y[m][t][c]) * sum_{t'*stride + k == t} src[(m*To + t')][k*C + c]
 __global__ void col2im_dact_kernel(const float* __restrict__ src, const float* __restrict__ y, float* __restrict__ dst, int64_t rows,
-                                   int Tin, int C, int ldc, int To, int ksz, int stride) {
+                                   int Tin, int C, int ldc, int To, int ksz, int stride, int act) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   int64_t total = rows * Tin * ldc;
   if (i >= total) return;
@@ -195,7 +198,7 @@ __global__ void col2im_dact_kernel(const float* __restrict__ src, const float* _
       s += src[(m * To + to) * (int64_t)(ksz * ldc) + k * ldc + c];
     }
     float yy = y[i];
-    s *= (yy > 0.0f ? 1.0f : yy + 1.0f);
+    s *= act_dy(act, yy);
   }
   dst[i] = s;
 }
@@ -219,12 +222,12 @@ static int hist_forward(const DwbcNetCfg& n, const float* P, const float* obs, c
   zero_cols_kernel<<<(unsigned)(((int64_t)rows * T * 2 + 255) / 256), 256, 0, st>>>(p.hproj, (int64_t)rows * T, 32, 30);
   zero_cols_kernel<<<(unsigned)(((int64_t)rows * 3 * 2 + 255) / 256), 256, 0, st>>>(p.hc2, (int64_t)rows * 3, 12, 10);
   RowMat hist = rowmat_grouped(obs + (n.num_obs - T * n.num_prop), idx, T, obs_stride, n.num_prop);
-  TRY(linear_fwd(hist, P + n.off_hist_w[0], n.num_prop, P + n.off_hist_b[0], p.hproj, 32, rows * T, 30, n.num_prop, ACT_ELU, 0, st));  // AC:80
+  TRY(linear_fwd(hist, P + n.off_hist_w[0], n.num_prop, P + n.off_hist_b[0], p.hproj, 32, rows * T, 30, n.num_prop, hid(n), 0, st));  // AC:80
   RowMat a1 = rowmat_grouped(p.hproj, nullptr, 4, (int64_t)T * 32, 2 * 32);
-  TRY(linear_fwd(a1, p.hw1, 128, P + n.off_hist_b[1], p.hc1, 20, rows * 4, 20, 128, ACT_ELU, 0, st));                                  // AC:59
+  TRY(linear_fwd(a1, p.hw1, 128, P + n.off_hist_b[1], p.hc1, 20, rows * 4, 20, 128, hid(n), 0, st));                                  // AC:59
   RowMat a2 = rowmat_grouped(p.hc1, nullptr, 3, 80, 20);
-  TRY(linear_fwd(a2, p.hw2, 40, P + n.off_hist_b[2], p.hc2, 12, rows * 3, 10, 40, ACT_ELU, 0, st));                                     // AC:60
-  TRY(linear_fwd(rowmat(p.hc2, 36), p.hwl, 36, P + n.off_hist_b[3], p.zh, Lld, rows, L, 36, ACT_ELU, 0, st));                           // AC:72
+  TRY(linear_fwd(a2, p.hw2, 40, P + n.off_hist_b[2], p.hc2, 12, rows * 3, 10, 40, hid(n), 0, st));                                     // AC:60
+  TRY(linear_fwd(rowmat(p.hc2, 36), p.hwl, 36, P + n.off_hist_b[3], p.zh, Lld, rows, L, 36, hid(n), 0, st));                           // AC:72
   return DWBC_OK;
 }
 
@@ -243,7 +246,7 @@ static int hist_latent_only(const DwbcNetCfg& n, const float* P, const float* ob
   a.w2 = P + n.off_hist_w[2]; a.b2 = P + n.off_hist_b[2]; a.wl = P + n.off_hist_w[3]; a.bl = P + n.off_hist_b[3];
   a.hist = rowmat_gather(obs + (n.num_obs - n.num_hist * n.num_prop), idx, obs_stride);
   a.out = out; a.ld_out = ld_out; a.rows = rows; a.latent = p.latent;
-  return launch_hist_fused(a, st);
+  return launch_hist_fused(a, hid(n), st);
 }
 
 static int priv_forward(const DwbcNetCfg& n, const float* P, const float* obs, const int64_t* idx, int64_t obs_stride, int rows,
@@ -252,7 +255,7 @@ static int priv_forward(const DwbcNetCfg& n, const float* P, const float* obs, c
   int in = n.num_priv;
   for (int l = 0; l < n.n_priv_layers; ++l) {
     int out = n.priv_dims[l], ld = (int)align_up(out, 4);
-    TRY(linear_fwd(h, P + n.off_priv_w[l], in, P + n.off_priv_b[l], p.priv[l], ld, rows, out, in, ACT_ELU, 0, st));  // AC:219-221
+    TRY(linear_fwd(h, P + n.off_priv_w[l], in, P + n.off_priv_b[l], p.priv[l], ld, rows, out, in, hid(n), 0, st));  // AC:219-221
     h = rowmat(p.priv[l], ld);
     in = out;
   }
@@ -260,9 +263,9 @@ static int priv_forward(const DwbcNetCfg& n, const float* P, const float* obs, c
 }
 
 static int head_forward(const float* P, RowMat h, int in, int nl, const int32_t* dims, int n_out, const int64_t* ow, const int64_t* ob,
-                        float* const* acts, float* out, int64_t ldo, int last_act, int rows, cudaStream_t st) {
+                        float* const* acts, float* out, int64_t ldo, int hact, int last_act, int rows, cudaStream_t st) {
   for (int l = 0; l < nl; ++l) {
-    TRY(linear_fwd(h, P + ow[l], in, P + ob[l], acts[l], dims[l], rows, dims[l], in, ACT_ELU, 0, st));
+    TRY(linear_fwd(h, P + ow[l], in, P + ob[l], acts[l], dims[l], rows, dims[l], in, hact, 0, st));
     h = rowmat(acts[l], dims[l]);
     in = dims[l];
   }
@@ -278,16 +281,16 @@ static int actor_forward(const DwbcNetCfg& n, const float* P, const float* obs, 
   int single = n.n_actor_layers;
   TRY(linear_fwd(x, P + n.off_actor_w[0], in0, P + n.off_actor_b[0], p.ab[0], n.actor_dims[0], rows, n.actor_dims[0], n.num_prop, ACT_NONE, 0, st));
   TRY(linear_fwd(rowmat(z, zld), P + n.off_actor_w[0] + n.num_prop, in0, nullptr, p.ab[0], n.actor_dims[0], rows, n.actor_dims[0], p.latent,
-                 ACT_ELU, 1, st));
+                 hid(n), 1, st));
   RowMat h = rowmat(p.ab[0], n.actor_dims[0]);
   int in = n.actor_dims[0];
   for (int l = 1; l < single; ++l) {
-    TRY(linear_fwd(h, P + n.off_actor_w[l], in, P + n.off_actor_b[l], p.ab[l], n.actor_dims[l], rows, n.actor_dims[l], in, ACT_ELU, 0, st));
+    TRY(linear_fwd(h, P + n.off_actor_w[l], in, P + n.off_actor_b[l], p.ab[l], n.actor_dims[l], rows, n.actor_dims[l], in, hid(n), 0, st));
     h = rowmat(p.ab[l], n.actor_dims[l]);
     in = n.actor_dims[l];
   }
-  TRY(head_forward(P, h, in, n.n_leg_layers, n.leg_dims, n.n_leg, n.off_aleg_w, n.off_aleg_b, p.al, p.mean, p.mean_ld, ACT_TANH, rows, st));
-  TRY(head_forward(P, h, in, n.n_arm_layers, n.arm_dims, n.n_arm, n.off_aarm_w, n.off_aarm_b, p.aa, p.mean + n.n_leg, p.mean_ld, ACT_TANH, rows, st));
+  TRY(head_forward(P, h, in, n.n_leg_layers, n.leg_dims, n.n_leg, n.off_aleg_w, n.off_aleg_b, p.al, p.mean, p.mean_ld, hid(n), ACT_TANH, rows, st));
+  TRY(head_forward(P, h, in, n.n_arm_layers, n.arm_dims, n.n_arm, n.off_aarm_w, n.off_aarm_b, p.aa, p.mean + n.n_leg, p.mean_ld, hid(n), ACT_TANH, rows, st));
   return DWBC_OK;
 }
 
@@ -297,12 +300,12 @@ static int critic_forward(const DwbcNetCfg& n, const float* P, const float* obs,
   RowMat h = rowmat_gather(obs, idx, obs_stride);
   int in = n.num_prop + n.num_priv;
   for (int l = 0; l < n.n_critic_layers; ++l) {
-    TRY(linear_fwd(h, P + n.off_critic_w[l], in, P + n.off_critic_b[l], p.cb[l], n.critic_dims[l], rows, n.critic_dims[l], in, ACT_ELU, 0, st));
+    TRY(linear_fwd(h, P + n.off_critic_w[l], in, P + n.off_critic_b[l], p.cb[l], n.critic_dims[l], rows, n.critic_dims[l], in, hid(n), 0, st));
     h = rowmat(p.cb[l], n.critic_dims[l]);
     in = n.critic_dims[l];
   }
-  TRY(head_forward(P, h, in, n.n_leg_layers, n.leg_dims, 1, n.off_cleg_w, n.off_cleg_b, p.cl, value, 2, ACT_NONE, rows, st));
-  TRY(head_forward(P, h, in, n.n_arm_layers, n.arm_dims, 1, n.off_carm_w, n.off_carm_b, p.ca, value + 1, 2, ACT_NONE, rows, st));
+  TRY(head_forward(P, h, in, n.n_leg_layers, n.leg_dims, 1, n.off_cleg_w, n.off_cleg_b, p.cl, value, 2, hid(n), ACT_NONE, rows, st));
+  TRY(head_forward(P, h, in, n.n_arm_layers, n.arm_dims, 1, n.off_carm_w, n.off_carm_b, p.ca, value + 1, 2, hid(n), ACT_NONE, rows, st));
   return DWBC_OK;
 }
 
@@ -328,10 +331,11 @@ static bool chain_usable(const DwbcNetCfg& n, const Plan& p, const float* obs, i
 
 // one head: optional trunk reload (the second head of a program), hidden layers in place, narrow last layer with its epilogue hook
 static void chain_head(C2Builder& b, const float* P, const float* trunk, int trunk_ld, bool reload, int in, int nl, const int32_t* dims, int n_out,
-                       const int64_t* ow, const int64_t* ob, float* const* acts, bool store, float* out, int64_t ldo, int last_act, int fin, int fin_c) {
+                       const int64_t* ow, const int64_t* ob, float* const* acts, bool store, float* out, int64_t ldo, int hact, int last_act, int fin,
+                       int fin_c) {
   if (reload) b.load(act_mat(trunk, trunk_ld), in, 0, pad8(in), b.pr.n_ops);
   for (int l = 0; l < nl; ++l) {
-    b.fwd(P + ow[l], in, P + ob[l], dims[l], ACT_ELU, 0, pad8(in), 1, C2PackSeg{0, 0, in}, C2PackSeg{0, 0, 0}, 0, store ? acts[l] : nullptr, dims[l],
+    b.fwd(P + ow[l], in, P + ob[l], dims[l], hact, 0, pad8(in), 1, C2PackSeg{0, 0, in}, C2PackSeg{0, 0, 0}, 0, store ? acts[l] : nullptr, dims[l],
           FIN_NONE, 0, store && img_dim(dims[l]));
     in = dims[l];
   }
@@ -358,22 +362,22 @@ static int build_forward(const DwbcNetCfg& n, const float* P, const float* obs, 
         B.load(rowmat(z_hist, zld), p.latent, 0, 32, 0);
       } else {
         B.load(rowmat_gather(obs + n.num_prop, idx, obs_stride), n.num_priv, C2_COL_PRIV, C2_COL_PRIV + pad8(n.num_priv), 0);
-        B.fwd(P + n.off_priv_w[0], n.num_priv, P + n.off_priv_b[0], n.priv_dims[0], ACT_ELU, C2_COL_PRIV, pad8(n.num_priv), 1,      // AC:219-221
+        B.fwd(P + n.off_priv_w[0], n.num_priv, P + n.off_priv_b[0], n.priv_dims[0], hid(n), C2_COL_PRIV, pad8(n.num_priv), 1,      // AC:219-221
               C2PackSeg{0, 0, n.num_priv}, C2PackSeg{0, 0, 0}, C2_COL_HID, store ? p.priv[0] : nullptr, align_up(n.priv_dims[0], 4));
-        B.fwd(P + n.off_priv_w[1], n.priv_dims[0], P + n.off_priv_b[1], p.latent, ACT_ELU, C2_COL_HID, pad8(n.priv_dims[0]), 1,
+        B.fwd(P + n.off_priv_w[1], n.priv_dims[0], P + n.off_priv_b[1], p.latent, hid(n), C2_COL_HID, pad8(n.priv_dims[0]), 1,
               C2PackSeg{0, 0, n.priv_dims[0]}, C2PackSeg{0, 0, 0}, 0, store ? p.priv[1] : nullptr, Lld, fin_mode == 2 ? FIN_REG : FIN_NONE, 0);
         first_main = 2;
       }
       const int k0 = pad8(C2_COL_PROP + n.num_prop);
       B.load(rowmat_gather(obs, idx, obs_stride), n.num_prop, C2_COL_PROP, k0, first_main);
       // backbone layer 0 over cat([obs_prop, z]) (AC:211): z occupies tile columns [0, latent), obs_prop [32, 32 + num_prop)
-      B.fwd(P + n.off_actor_w[0], in0, P + n.off_actor_b[0], n.actor_dims[0], ACT_ELU, 0, k0, 2, C2PackSeg{0, n.num_prop, p.latent},
+      B.fwd(P + n.off_actor_w[0], in0, P + n.off_actor_b[0], n.actor_dims[0], hid(n), 0, k0, 2, C2PackSeg{0, n.num_prop, p.latent},
             C2PackSeg{C2_COL_PROP, 0, n.num_prop}, 0, (store || (keep && na == 1)) ? p.ab[0] : nullptr, n.actor_dims[0], FIN_NONE, 0,
             img_dim(n.actor_dims[0]) && (store || (keep && na == 1)));
       int in = n.actor_dims[0];
       for (int l = 1; l < na; ++l) {                                                   // AC:211-213
         const bool st = store || (keep && l == na - 1);
-        B.fwd(P + n.off_actor_w[l], in, P + n.off_actor_b[l], n.actor_dims[l], ACT_ELU, 0, pad8(in), 1, C2PackSeg{0, 0, in}, C2PackSeg{0, 0, 0}, 0,
+        B.fwd(P + n.off_actor_w[l], in, P + n.off_actor_b[l], n.actor_dims[l], hid(n), 0, pad8(in), 1, C2PackSeg{0, 0, in}, C2PackSeg{0, 0, 0}, 0,
               st ? p.ab[l] : nullptr, n.actor_dims[l], FIN_NONE, 0, img_dim(n.actor_dims[l]) && st);
         in = n.actor_dims[l];
       }
@@ -382,11 +386,11 @@ static int build_forward(const DwbcNetCfg& n, const float* P, const float* obs, 
     const int fin = fin_mode == 2 ? FIN_PPO : (fin_mode == 1 ? FIN_ACT : FIN_NONE);
     float* mean = fin_mode == 0 ? p.mean : nullptr;
     const int in = common(*A, A2 == nullptr);
-    chain_head(*A, P, p.ab[na - 1], in, false, in, n.n_leg_layers, n.leg_dims, n.n_leg, n.off_aleg_w, n.off_aleg_b, p.al, store, mean, p.mean_ld, ACT_TANH, fin, 0);
+    chain_head(*A, P, p.ab[na - 1], in, false, in, n.n_leg_layers, n.leg_dims, n.n_leg, n.off_aleg_w, n.off_aleg_b, p.al, store, mean, p.mean_ld, hid(n), ACT_TANH, fin, 0);
     C2Builder& Barm = A2 ? *A2 : *A;
     if (A2) common(*A2, false);
     chain_head(Barm, P, p.ab[na - 1], in, A2 == nullptr, in, n.n_arm_layers, n.arm_dims, n.n_arm, n.off_aarm_w, n.off_aarm_b, p.aa, store,
-               mean ? mean + n.n_leg : nullptr, p.mean_ld, ACT_TANH, fin, 1);
+               mean ? mean + n.n_leg : nullptr, p.mean_ld, hid(n), ACT_TANH, fin, 1);
     A->finish();
     if (A2) A2->finish();
     if (!A->ok || (A2 && !A2->ok)) return DWBC_ERR_UNSUPPORTED;
@@ -398,7 +402,7 @@ static int build_forward(const DwbcNetCfg& n, const float* P, const float* obs, 
       B.load(rowmat_gather(obs, idx, obs_stride), in, 0, pad8(in), 0);
       for (int l = 0; l < nc; ++l) {                                                   // AC:280-286
         const bool st = store || (keep && l == nc - 1);
-        B.fwd(P + n.off_critic_w[l], in, P + n.off_critic_b[l], n.critic_dims[l], ACT_ELU, 0, pad8(in), 1, C2PackSeg{0, 0, in}, C2PackSeg{0, 0, 0}, 0,
+        B.fwd(P + n.off_critic_w[l], in, P + n.off_critic_b[l], n.critic_dims[l], hid(n), 0, pad8(in), 1, C2PackSeg{0, 0, in}, C2PackSeg{0, 0, 0}, 0,
               st ? p.cb[l] : nullptr, n.critic_dims[l], FIN_NONE, 0, img_dim(n.critic_dims[l]) && st);
         in = n.critic_dims[l];
       }
@@ -406,11 +410,11 @@ static int build_forward(const DwbcNetCfg& n, const float* P, const float* obs, 
     };
     const int fin = fin_mode == 2 ? FIN_VALUE : FIN_NONE;
     const int in = common(*C, C2 == nullptr);
-    chain_head(*C, P, p.cb[nc - 1], in, false, in, n.n_leg_layers, n.leg_dims, 1, n.off_cleg_w, n.off_cleg_b, p.cl, store, value, 2, ACT_NONE, fin, 0);
+    chain_head(*C, P, p.cb[nc - 1], in, false, in, n.n_leg_layers, n.leg_dims, 1, n.off_cleg_w, n.off_cleg_b, p.cl, store, value, 2, hid(n), ACT_NONE, fin, 0);
     C2Builder& Barm = C2 ? *C2 : *C;
     if (C2) common(*C2, false);
     chain_head(Barm, P, p.cb[nc - 1], in, C2 == nullptr, in, n.n_arm_layers, n.arm_dims, 1, n.off_carm_w, n.off_carm_b, p.ca, store,
-               value + 1, 2, ACT_NONE, fin, 1);
+               value + 1, 2, hid(n), ACT_NONE, fin, 1);
     C->finish();
     if (C2) C2->finish();
     if (!C->ok || (C2 && !C2->ok)) return DWBC_ERR_UNSUPPORTED;
@@ -571,9 +575,9 @@ __global__ void __launch_bounds__(128) ppo_loss_kernel(const LossArgs a) {
   if (threadIdx.x < a.n_act) atomicAdd(a.grad_std + threadIdx.x, sred[threadIdx.x]);
 }
 
-// DAgger loss PPO:273-276: mean_rows || sg(zp) - zh ||_2 ; writes d/d zh_pre (ELU' folded in)
+// DAgger loss PPO:273-276: mean_rows || sg(zp) - zh ||_2 ; writes d/d zh_pre (the activation derivative folded in)
 __global__ void __launch_bounds__(128) dagger_loss_kernel(const float* __restrict__ zp, const float* __restrict__ zh, int zld, int latent,
-                                                          float* __restrict__ g, float* __restrict__ loss, int rows) {
+                                                          float* __restrict__ g, float* __restrict__ loss, int rows, int act) {
   __shared__ float red[4];
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   float l = 0.0f;
@@ -588,7 +592,7 @@ __global__ void __launch_bounds__(128) dagger_loss_kernel(const float* __restric
     const float s = nrm > 0.0f ? 1.0f / ((float)rows * nrm) : 0.0f;
     for (int i = 0; i < latent; ++i) {
       const float y = zh[(int64_t)r * zld + i];
-      g[(int64_t)r * zld + i] = -s * (zp[(int64_t)r * zld + i] - y) * (y > 0.0f ? 1.0f : y + 1.0f);
+      g[(int64_t)r * zld + i] = -s * (zp[(int64_t)r * zld + i] - y) * act_dy(act, y);
     }
   }
   float s = warp_sum(l);
@@ -598,12 +602,12 @@ __global__ void __launch_bounds__(128) dagger_loss_kernel(const float* __restric
 }
 
 // ---- backward -----------------------------------------------------------------------------------
-// Backward of one head: Linear(+ELU) x nl, then Linear -> out.  G_out = d/d(pre-activation of the
+// Backward of one head: Linear(+act) x nl, then Linear -> out.  G_out = d/d(pre-activation of the
 // last layer) [rows, n_out].  Accumulates weight grads into `grad`, and adds the head's
-// contribution to d(backbone output) into dtrunk (beta_trunk; ELU' of the trunk applied if apply_dact).
+// contribution to d(backbone output) into dtrunk (beta_trunk; act' of the trunk applied if apply_dact).
 static int head_backward(const float* P, float* grad, RowMat G_out, int n_out, int nl, const int32_t* dims, const int64_t* ow,
                          const int64_t* ob, float* const* acts, RowMat trunk, int trunk_dim, float* dtrunk, int beta_trunk,
-                         int apply_dact, float* dA, float* dB, int rows, cudaStream_t st) {
+                         int apply_dact, float* dA, float* dB, int hact, int rows, cudaStream_t st) {
   RowMat G = G_out;
   int gout = n_out;
   for (int l = nl; l >= 0; --l) {
@@ -611,10 +615,10 @@ static int head_backward(const float* P, float* grad, RowMat G_out, int n_out, i
     RowMat X = l == 0 ? trunk : rowmat(acts[l - 1], dims[l - 1]);
     TRY(linear_bwd_weight(G, X, grad + ow[l], in, grad + ob[l], rows, gout, in, st));
     if (l == 0) {
-      TRY(linear_bwd_data(G, P + ow[l], in, dtrunk, trunk_dim, rows, in, gout, apply_dact ? ACT_ELU : ACT_NONE, trunk, beta_trunk, st));
+      TRY(linear_bwd_data(G, P + ow[l], in, dtrunk, trunk_dim, rows, in, gout, apply_dact ? hact : ACT_NONE, trunk, beta_trunk, st));
     } else {
       float* d = (l & 1) ? dA : dB;
-      TRY(linear_bwd_data(G, P + ow[l], in, d, in, rows, in, gout, ACT_ELU, X, 0, st));
+      TRY(linear_bwd_data(G, P + ow[l], in, d, in, rows, in, gout, hact, X, 0, st));
       G = rowmat(d, in);
       gout = in;
     }
@@ -629,9 +633,9 @@ struct HeadDesc { int nl; const int32_t* dims; const int64_t* ow; const int64_t*
 
 // data-gradient ops of one head, last layer first.  The head's loss gradient [rows, g_ld] is loaded into tile columns [0, g_ld) right
 // before its first op; column g_col + j of that window multiplies row j of the last layer's weights.  The trunk gradient of the
-// FIRST head goes to `scratch` unactivated; the second head adds it and applies the trunk's ELU'.
+// FIRST head goes to `scratch` unactivated; the second head adds it and applies the trunk's act'.
 static void chain_head_bwd(C2Builder& b, const float* P, const HeadDesc& hd, const float* g, int g_ld, int g_col, int trunk_dim, const float* trunk,
-                           bool second, float* scratch, float* dz_trunk) {
+                           bool second, float* scratch, float* dz_trunk, int hact) {
   b.load(rowmat(g, g_ld), g_ld, 0, pad8(g_ld), b.pr.n_ops);
   for (int l = hd.nl; l >= 0; --l) {
     const int in = l == 0 ? trunk_dim : hd.dims[l - 1];
@@ -640,11 +644,11 @@ static void chain_head_bwd(C2Builder& b, const float* P, const HeadDesc& hd, con
     const int kpad = narrow ? pad8(g_ld) : pad8(out);
     const C2PackSeg seg{narrow ? g_col : 0, 0, out};
     if (l > 0)
-      b.bwd(P + hd.ow[l], in, in, 0, kpad, seg, ACT_ELU, hd.acts[l - 1], in, nullptr, 0, 0, hd.dz[l - 1], in, img_dim(in), img_dim(in));
+      b.bwd(P + hd.ow[l], in, in, 0, kpad, seg, hact, hd.acts[l - 1], in, nullptr, 0, 0, hd.dz[l - 1], in, img_dim(in), img_dim(in));
     else if (!second)
       b.bwd(P + hd.ow[0], in, in, 0, kpad, seg, ACT_NONE, nullptr, 0, nullptr, 0, -1, scratch, trunk_dim);
     else
-      b.bwd(P + hd.ow[0], in, in, 0, kpad, seg, ACT_ELU, trunk, trunk_dim, scratch, trunk_dim, 0, dz_trunk, trunk_dim, img_dim(trunk_dim), img_dim(trunk_dim));
+      b.bwd(P + hd.ow[0], in, in, 0, kpad, seg, hact, trunk, trunk_dim, scratch, trunk_dim, 0, dz_trunk, trunk_dim, img_dim(trunk_dim), img_dim(trunk_dim));
   }
 }
 
@@ -675,27 +679,27 @@ static int build_backward(const DwbcNetCfg& n, const float* P, const Plan& p, C2
   const BwdDescs d = bwd_descs(n, p);
   // ---- critic: both value heads read their column of the [rows, 4] value-gradient buffer ----
   const int cnb = n.n_critic_layers, ctd = n.critic_dims[cnb - 1];
-  chain_head_bwd(C, P, d.cl, p.g_vl, 4, 0, ctd, p.cb[cnb - 1], false, p.d1, nullptr);
-  chain_head_bwd(C, P, d.ca, p.g_vl, 4, 1, ctd, p.cb[cnb - 1], true, p.d1, p.dzc_b[cnb - 1]);
+  chain_head_bwd(C, P, d.cl, p.g_vl, 4, 0, ctd, p.cb[cnb - 1], false, p.d1, nullptr, hid(n));
+  chain_head_bwd(C, P, d.ca, p.g_vl, 4, 1, ctd, p.cb[cnb - 1], true, p.d1, p.dzc_b[cnb - 1], hid(n));
   for (int l = cnb - 1; l >= 1; --l)
-    C.bwd(P + n.off_critic_w[l], n.critic_dims[l - 1], n.critic_dims[l - 1], 0, pad8(n.critic_dims[l]), C2PackSeg{0, 0, n.critic_dims[l]}, ACT_ELU,
+    C.bwd(P + n.off_critic_w[l], n.critic_dims[l - 1], n.critic_dims[l - 1], 0, pad8(n.critic_dims[l]), C2PackSeg{0, 0, n.critic_dims[l]}, hid(n),
           p.cb[l - 1], n.critic_dims[l - 1], nullptr, 0, 0, p.dzc_b[l - 1], n.critic_dims[l - 1], img_dim(n.critic_dims[l - 1]), img_dim(n.critic_dims[l - 1]));
   C.finish();
   // ---- actor + privileged encoder ----
   const int anb = n.n_actor_layers, atd = n.actor_dims[anb - 1];
-  chain_head_bwd(A, P, d.al, p.g_leg, gleg_ld, 0, atd, p.ab[anb - 1], false, p.d0, nullptr);
-  chain_head_bwd(A, P, d.aa, p.g_arm, garm_ld, 0, atd, p.ab[anb - 1], true, p.d0, p.dza_b[anb - 1]);
+  chain_head_bwd(A, P, d.al, p.g_leg, gleg_ld, 0, atd, p.ab[anb - 1], false, p.d0, nullptr, hid(n));
+  chain_head_bwd(A, P, d.aa, p.g_arm, garm_ld, 0, atd, p.ab[anb - 1], true, p.d0, p.dza_b[anb - 1], hid(n));
   for (int l = anb - 1; l >= 1; --l)
-    A.bwd(P + n.off_actor_w[l], n.actor_dims[l - 1], n.actor_dims[l - 1], 0, pad8(n.actor_dims[l]), C2PackSeg{0, 0, n.actor_dims[l]}, ACT_ELU,
+    A.bwd(P + n.off_actor_w[l], n.actor_dims[l - 1], n.actor_dims[l - 1], 0, pad8(n.actor_dims[l]), C2PackSeg{0, 0, n.actor_dims[l]}, hid(n),
           p.ab[l - 1], n.actor_dims[l - 1], nullptr, 0, 0, p.dza_b[l - 1], n.actor_dims[l - 1], img_dim(n.actor_dims[l - 1]), img_dim(n.actor_dims[l - 1]));
   const int in0 = n.num_prop + p.latent, np = n.n_priv_layers;
   float* z = p.priv[np - 1];
-  // dL/dz = policy path through the latent columns of backbone layer 0 + privileged-latent regulariser (g_z), through the encoder's last ELU
-  A.bwd(P + n.off_actor_w[0] + n.num_prop, in0, p.latent, 0, pad8(n.actor_dims[0]), C2PackSeg{0, 0, n.actor_dims[0]}, ACT_ELU, z, Lld, p.g_z, Lld, 0,
+  // dL/dz = policy path through the latent columns of backbone layer 0 + privileged-latent regulariser (g_z), through the encoder's last activation
+  A.bwd(P + n.off_actor_w[0] + n.num_prop, in0, p.latent, 0, pad8(n.actor_dims[0]), C2PackSeg{0, 0, n.actor_dims[0]}, hid(n), z, Lld, p.g_z, Lld, 0,
         p.dzp[np - 1], Lld);
   for (int l = np - 1; l >= 1; --l) {
     const int in = n.priv_dims[l - 1], ldin = (int)align_up(in, 4);
-    A.bwd(P + n.off_priv_w[l], in, in, 0, pad8(n.priv_dims[l]), C2PackSeg{0, 0, n.priv_dims[l]}, ACT_ELU, p.priv[l - 1], ldin, nullptr, 0, l - 1 > 0 ? 0 : -1,
+    A.bwd(P + n.off_priv_w[l], in, in, 0, pad8(n.priv_dims[l]), C2PackSeg{0, 0, n.priv_dims[l]}, hid(n), p.priv[l - 1], ldin, nullptr, 0, l - 1 > 0 ? 0 : -1,
           p.dzp[l - 1], ldin);
   }
   A.finish();
@@ -894,9 +898,9 @@ extern "C" int dwbc_ppo_minibatch_grad(const DwbcNetCfg* net, const float* param
     const int nb = n.n_critic_layers, tdim = n.critic_dims[nb - 1];
     RowMat trunk = rowmat(p.cb[nb - 1], tdim);
     TRY(head_backward(P, grad, rowmat(p.g_vl, 4), 1, n.n_leg_layers, n.leg_dims, n.off_cleg_w, n.off_cleg_b, p.cl, trunk, tdim, p.d2, 0, 0,
-                      p.d0, p.d1, rows, st));
+                      p.d0, p.d1, hid(n), rows, st));
     TRY(head_backward(P, grad, rowmat(p.g_va, 4), 1, n.n_arm_layers, n.arm_dims, n.off_carm_w, n.off_carm_b, p.ca, trunk, tdim, p.d2, 1, 1,
-                      p.d0, p.d1, rows, st));
+                      p.d0, p.d1, hid(n), rows, st));
     RowMat G = rowmat(p.d2, tdim);
     int gout = tdim;
     for (int l = nb - 1; l >= 0; --l) {
@@ -905,7 +909,7 @@ extern "C" int dwbc_ppo_minibatch_grad(const DwbcNetCfg* net, const float* param
       TRY(linear_bwd_weight(G, X, grad + n.off_critic_w[l], in, grad + n.off_critic_b[l], rows, gout, in, st));
       if (l > 0) {
         float* d = (l & 1) ? p.d0 : p.d1;
-        TRY(linear_bwd_data(G, P + n.off_critic_w[l], in, d, in, rows, in, gout, ACT_ELU, X, 0, st));
+        TRY(linear_bwd_data(G, P + n.off_critic_w[l], in, d, in, rows, in, gout, hid(n), X, 0, st));
         G = rowmat(d, in);
         gout = in;
       }
@@ -916,9 +920,9 @@ extern "C" int dwbc_ppo_minibatch_grad(const DwbcNetCfg* net, const float* param
     const int nb = n.n_actor_layers, tdim = n.actor_dims[nb - 1];
     RowMat trunk = rowmat(p.ab[nb - 1], tdim);
     TRY(head_backward(P, grad, rowmat(p.g_leg, gleg_ld), n.n_leg, n.n_leg_layers, n.leg_dims, n.off_aleg_w, n.off_aleg_b, p.al, trunk, tdim,
-                      p.d2, 0, 0, p.d0, p.d1, rows, st));
+                      p.d2, 0, 0, p.d0, p.d1, hid(n), rows, st));
     TRY(head_backward(P, grad, rowmat(p.g_arm, garm_ld), n.n_arm, n.n_arm_layers, n.arm_dims, n.off_aarm_w, n.off_aarm_b, p.aa, trunk, tdim,
-                      p.d2, 1, 1, p.d0, p.d1, rows, st));
+                      p.d2, 1, 1, p.d0, p.d1, hid(n), rows, st));
     RowMat G = rowmat(p.d2, tdim);
     int gout = tdim;
     for (int l = nb - 1; l >= 1; --l) {
@@ -926,7 +930,7 @@ extern "C" int dwbc_ppo_minibatch_grad(const DwbcNetCfg* net, const float* param
       RowMat X = rowmat(p.ab[l - 1], in);
       TRY(linear_bwd_weight(G, X, grad + n.off_actor_w[l], in, grad + n.off_actor_b[l], rows, gout, in, st));
       float* d = (l & 1) ? p.d0 : p.d1;
-      TRY(linear_bwd_data(G, P + n.off_actor_w[l], in, d, in, rows, in, gout, ACT_ELU, X, 0, st));
+      TRY(linear_bwd_data(G, P + n.off_actor_w[l], in, d, in, rows, in, gout, hid(n), X, 0, st));
       G = rowmat(d, in);
       gout = in;
     }
@@ -935,8 +939,8 @@ extern "C" int dwbc_ppo_minibatch_grad(const DwbcNetCfg* net, const float* param
     TRY(linear_bwd_weight(G, rowmat_gather(s->observations, idx, s->obs_stride), grad + n.off_actor_w[0], in0, grad + n.off_actor_b[0], rows,
                           gout, n.num_prop, st));
     TRY(linear_bwd_weight(G, rowmat(z, Lld), grad + n.off_actor_w[0] + n.num_prop, in0, nullptr, rows, gout, p.latent, st));
-    // dL/dz = (policy path) + (priv-reg path, already in g_z); then through the ELU of the encoder's last layer
-    TRY(linear_bwd_data(G, P + n.off_actor_w[0] + n.num_prop, in0, p.g_z, Lld, rows, p.latent, gout, ACT_ELU, rowmat(z, Lld), 1, st));
+    // dL/dz = (policy path) + (priv-reg path, already in g_z); then through the activation of the encoder's last layer
+    TRY(linear_bwd_data(G, P + n.off_actor_w[0] + n.num_prop, in0, p.g_z, Lld, rows, p.latent, gout, hid(n), rowmat(z, Lld), 1, st));
     RowMat Gp = rowmat(p.g_z, Lld);
     int gp = p.latent;
     for (int l = n.n_priv_layers - 1; l >= 0; --l) {
@@ -946,7 +950,7 @@ extern "C" int dwbc_ppo_minibatch_grad(const DwbcNetCfg* net, const float* param
       TRY(linear_bwd_weight(Gp, X, grad + n.off_priv_w[l], in, grad + n.off_priv_b[l], rows, gp, in, st));
       if (l > 0) {
         float* d = (l & 1) ? p.d0 : p.d1;
-        TRY(linear_bwd_data(Gp, P + n.off_priv_w[l], in, d, ldin, rows, in, gp, ACT_ELU, X, 0, st));
+        TRY(linear_bwd_data(Gp, P + n.off_priv_w[l], in, d, ldin, rows, in, gp, hid(n), X, 0, st));
         Gp = rowmat(d, ldin);
         gp = in;
       }
@@ -971,19 +975,19 @@ extern "C" int dwbc_dagger_minibatch_grad(const DwbcNetCfg* net, const float* pa
   if (cudaMemsetAsync(p.dhwl, 0, sizeof(float) * (32 * 36), st) != cudaSuccess) return DWBC_ERR_LAUNCH;
   TRY(priv_forward(n, P, s->observations, idx, s->obs_stride, rows, p, st));             // PPO:273-274 (no grad)
   TRY(hist_forward(n, P, s->observations, idx, s->obs_stride, rows, p, st));             // PPO:275
-  dagger_loss_kernel<<<(rows + 127) / 128, 128, 0, st>>>(p.priv[n.n_priv_layers - 1], p.zh, Lld, L, p.dzh, losses_out, rows);
+  dagger_loss_kernel<<<(rows + 127) / 128, 128, 0, st>>>(p.priv[n.n_priv_layers - 1], p.zh, Lld, L, p.dzh, losses_out, rows, hid(n));
   DWBC_LAUNCH_CHECK();
-  // linear_output: zh = ELU(flat . Wl'^T + b)
+  // linear_output: zh = act(flat . Wl'^T + b)
   RowMat G4 = rowmat(p.dzh, Lld);
   TRY(linear_bwd_weight(G4, rowmat(p.hc2, 36), p.dhwl, 36, grad + n.off_hist_b[3], rows, L, 36, st));
-  TRY(linear_bwd_data(G4, p.hwl, 36, p.d0, 36, rows, 36, L, ACT_ELU, rowmat(p.hc2, 36), 0, st));    // d(conv2 pre-act) as [rows*3, 12]
+  TRY(linear_bwd_data(G4, p.hwl, 36, p.d0, 36, rows, 36, L, hid(n), rowmat(p.hc2, 36), 0, st));    // d(conv2 pre-act) as [rows*3, 12]
   // conv2
   RowMat G3 = rowmat(p.d0, 12);
   TRY(linear_bwd_weight(G3, rowmat_grouped(p.hc1, nullptr, 3, 80, 20), p.dhw2, 40, grad + n.off_hist_b[2], rows * 3, 10, 40, st));
   TRY(linear_bwd_data(G3, p.hw2, 40, p.dh_a2, 40, rows * 3, 40, 10, ACT_NONE, RowMat{}, 0, st));
   {
     int64_t tot = (int64_t)rows * 4 * 20;
-    col2im_dact_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(p.dh_a2, p.hc1, p.dh_c1, rows, 4, 20, 20, 3, 2, 1);
+    col2im_dact_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(p.dh_a2, p.hc1, p.dh_c1, rows, 4, 20, 20, 3, 2, 1, hid(n));
     DWBC_LAUNCH_CHECK();
   }
   // conv1
@@ -992,7 +996,7 @@ extern "C" int dwbc_dagger_minibatch_grad(const DwbcNetCfg* net, const float* pa
   TRY(linear_bwd_data(G2, p.hw1, 128, p.dh_a1, 128, rows * 4, 128, 20, ACT_NONE, RowMat{}, 0, st));
   {
     int64_t tot = (int64_t)rows * T * 32;
-    col2im_dact_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(p.dh_a1, p.hproj, p.dh_proj, rows, T, 30, 32, 4, 4, 2);
+    col2im_dact_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(p.dh_a1, p.hproj, p.dh_proj, rows, T, 30, 32, 4, 4, 2, hid(n));
     DWBC_LAUNCH_CHECK();
   }
   // projection
@@ -1009,6 +1013,7 @@ extern "C" int dwbc_dagger_minibatch_grad(const DwbcNetCfg* net, const float* pa
 //   mode 0: Y[M,N] = act(X[M,K] W[N,K]^T + b)      mode 1: dX[M,N] = G[M,K] W[K,N]      mode 2: dW[M,N] += G[K,M]^T X[K,N], db += colsum(G)
 extern "C" int dwbc_debug_gemm(int mode, int tc, const float* A, int64_t lda, const float* Bm, int64_t ldb, float* C, int64_t ldc,
                                const float* bias, float* dbias, int M, int N, int K, int act, dwbc_stream_t stream) {
+  if (act < 0 || act >= ACT_COUNT) return DWBC_ERR_ARG;
   const int saved = mlp_precision;
   mlp_precision = tc;
   int rc;

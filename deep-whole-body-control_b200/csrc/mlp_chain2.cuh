@@ -236,6 +236,7 @@ __device__ __forceinline__ void c2_upk(uint64_t p, float& a, float& b) { asm("mo
 __device__ __forceinline__ uint64_t c2_add2(uint64_t a, uint64_t b) { uint64_t r; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
 __device__ __forceinline__ uint64_t c2_sub2(uint64_t a, uint64_t b) { uint64_t r; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
 __device__ __forceinline__ uint64_t c2_mul2(uint64_t a, uint64_t b) { uint64_t r; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
+__device__ __forceinline__ uint64_t c2_fma2(uint64_t a, uint64_t b, uint64_t c) { uint64_t r; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c)); return r; }
 // 2^x, flush-to-zero form: ONE MUFU.EX2.  (__expf = ex2.approx.f32 of x * log2 e WITHOUT .ftz, which ptxas wraps in a range test and two
 // scaling multiplies per element for results in the denormal range -- irrelevant for e^x - 1.)
 __device__ __forceinline__ float c2_ex2(float x) { float r; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
@@ -248,8 +249,9 @@ __device__ __forceinline__ void c2_lo_chunk(float* v) {
   for (int jj = 0; jj < 32; jj += 2) c2_upk(c2_lo2(c2_pk(v[jj], v[jj + 1])), v[jj], v[jj + 1]);
 }
 
+// kAct == ACT_RELU stands for ReLU and leaky ReLU (negative-side `slope`)
 template <int kAct, bool kFull>
-__device__ __forceinline__ void c2_bias_act(float* v, const float* bias, int nvalid) {
+__device__ __forceinline__ void c2_bias_act(float* v, const float* bias, int nvalid, float slope = 0.0f) {
   const uint64_t l2e = c2_pk(C2_LOG2E, C2_LOG2E), m1 = c2_pk(-1.0f, -1.0f);
 #pragma unroll
   for (int j4 = 0; j4 < 8; ++j4) {
@@ -264,20 +266,37 @@ __device__ __forceinline__ void c2_bias_act(float* v, const float* bias, int nva
         c2_upk(c2_mul2(c2_pk(fminf(x0, 0.0f), fminf(x1, 0.0f)), l2e), e0, e1);
         c2_upk(c2_add2(c2_add2(c2_pk(c2_ex2(e0), c2_ex2(e1)), m1), c2_pk(fmaxf(x0, 0.0f), fmaxf(x1, 0.0f))), x0, x1);
       }
+      if (kAct == ACT_SELU) {       // lambda max(x,0) + lambda alpha (e^{min(x,0)} - 1): the ELU line with two scales
+        float e0, e1;
+        c2_upk(c2_mul2(c2_pk(fminf(x0, 0.0f), fminf(x1, 0.0f)), l2e), e0, e1);
+        c2_upk(c2_fma2(c2_add2(c2_pk(c2_ex2(e0), c2_ex2(e1)), m1), c2_pk(SELU_SCALE * SELU_ALPHA, SELU_SCALE * SELU_ALPHA),
+                       c2_mul2(c2_pk(fmaxf(x0, 0.0f), fmaxf(x1, 0.0f)), c2_pk(SELU_SCALE, SELU_SCALE))), x0, x1);
+      }
+      if (kAct == ACT_RELU) {       // ReLU and leaky ReLU: max(x,0) + slope min(x,0), slope = 0 / 0.01 (exact: one rounding)
+        c2_upk(c2_fma2(c2_pk(fminf(x0, 0.0f), fminf(x1, 0.0f)), c2_pk(slope, slope), c2_pk(fmaxf(x0, 0.0f), fmaxf(x1, 0.0f))), x0, x1);
+      }
       if (kAct == ACT_TANH) { x0 = t2_tanh(x0); x1 = t2_tanh(x1); }
+      if (kAct == ACT_SIGMOID) { x0 = __fdividef(1.0f, 1.0f + c2_ex2(-C2_LOG2E * x0)); x1 = __fdividef(1.0f, 1.0f + c2_ex2(-C2_LOG2E * x1)); }
       v[jj] = (kFull || jj < nvalid) ? x0 : 0.0f;
       v[jj + 1] = (kFull || jj + 1 < nvalid) ? x1 : 0.0f;
     }
   }
 }
 __device__ __forceinline__ void c2_bias_act_any(float* v, const float* bias, int act, int nvalid) {
+  const float slope = act == ACT_LRELU ? LRELU_SLOPE : 0.0f;
   if (nvalid >= 32) {
     if (act == ACT_ELU) c2_bias_act<ACT_ELU, true>(v, bias, 32);
     else if (act == ACT_TANH) c2_bias_act<ACT_TANH, true>(v, bias, 32);
+    else if (act == ACT_SELU) c2_bias_act<ACT_SELU, true>(v, bias, 32);
+    else if (act == ACT_RELU || act == ACT_LRELU) c2_bias_act<ACT_RELU, true>(v, bias, 32, slope);
+    else if (act == ACT_SIGMOID) c2_bias_act<ACT_SIGMOID, true>(v, bias, 32);
     else c2_bias_act<ACT_NONE, true>(v, bias, 32);
   } else {
     if (act == ACT_ELU) c2_bias_act<ACT_ELU, false>(v, bias, nvalid);
     else if (act == ACT_TANH) c2_bias_act<ACT_TANH, false>(v, bias, nvalid);
+    else if (act == ACT_SELU) c2_bias_act<ACT_SELU, false>(v, bias, nvalid);
+    else if (act == ACT_RELU || act == ACT_LRELU) c2_bias_act<ACT_RELU, false>(v, bias, nvalid, slope);
+    else if (act == ACT_SIGMOID) c2_bias_act<ACT_SIGMOID, false>(v, bias, nvalid);
     else c2_bias_act<ACT_NONE, false>(v, bias, nvalid);
   }
 }
@@ -781,11 +800,11 @@ __global__ void __launch_bounds__(C2_THREADS, 1) chain2_kernel(const __grid_cons
                   }
                 }
               }
-              if (use_x) {                                   // AC ELU / tanh derivatives from the layer's OUTPUTS
+              if (use_x) {                                   // activation derivatives from the layer's OUTPUTS
                 if (o.act == ACT_TANH) {
 #pragma unroll
                   for (int jj = 0; jj < 32; ++jj) v[jj] *= 1.0f - x[u][jj] * x[u][jj];
-                } else {                                     // ELU'(y) = y > 0 ? 1 : y + 1 = min(y + 1, 1), on pairs
+                } else if (o.act == ACT_ELU) {               // ELU'(y) = y > 0 ? 1 : y + 1 = min(y + 1, 1), on pairs
                   const uint64_t one2 = c2_pk(1.0f, 1.0f);
 #pragma unroll
                   for (int jj = 0; jj < 32; jj += 2) {
@@ -793,6 +812,15 @@ __global__ void __launch_bounds__(C2_THREADS, 1) chain2_kernel(const __grid_cons
                     c2_upk(c2_add2(c2_pk(x[u][jj], x[u][jj + 1]), one2), d0, d1);
                     c2_upk(c2_mul2(c2_pk(v[jj], v[jj + 1]), c2_pk(fminf(d0, 1.0f), fminf(d1, 1.0f))), v[jj], v[jj + 1]);
                   }
+                } else if (o.act == ACT_SIGMOID) {           // y (1 - y)
+#pragma unroll
+                  for (int jj = 0; jj < 32; ++jj) v[jj] *= x[u][jj] * (1.0f - x[u][jj]);
+                } else {                                     // SELU / ReLU / leaky ReLU: y > 0 ? p : q y + r
+                  const bool selu = o.act == ACT_SELU;
+                  const float p = selu ? SELU_SCALE : 1.0f, qq = selu ? 1.0f : 0.0f,
+                              rr = selu ? SELU_SCALE * SELU_ALPHA : (o.act == ACT_LRELU ? LRELU_SLOPE : 0.0f);
+#pragma unroll
+                  for (int jj = 0; jj < 32; ++jj) v[jj] *= x[u][jj] > 0.0f ? p : fmaf(qq, x[u][jj], rr);
                 }
               }
               if (o.N - c0 < 32) {                           // ragged last chunk: the pad columns are operand columns of the next op

@@ -86,7 +86,7 @@ extern "C" int dwbc_enforce_min_std(float* params, int64_t off_std, const float*
 unsigned long long dwbc_launch_counter = 0;
 extern "C" uint64_t dwbc_launch_count(void) { return dwbc_launch_counter; }
 
-extern "C" const char* dwbc_version(void) { return "dwbc-b200 0.1 (sm_100a, abi 3)"; }
+extern "C" const char* dwbc_version(void) { return "dwbc-b200 0.1 (sm_100a, abi 4)"; }
 
 extern "C" void dwbc_struct_sizes(int64_t out[6]) {
   out[0] = sizeof(DwbcEnvCfg); out[1] = sizeof(DwbcEnvBuffers); out[2] = sizeof(DwbcStepArgs);

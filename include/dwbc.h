@@ -33,7 +33,7 @@ enum {
   DWBC_ERR_LAUNCH = -3       /* cudaGetLastError() != cudaSuccess after the launch */
 };
 
-#define DWBC_ABI_VERSION 3
+#define DWBC_ABI_VERSION 4
 #define DWBC_MAX_DOF 24
 #define DWBC_MAX_TERMS 40   /* active reward terms per channel */
 #define DWBC_MAX_IDX 8      /* penalised / termination contact bodies */
@@ -234,6 +234,18 @@ int dwbc_normalize_advantages(float* advantages, const double* stats, int64_t co
 
 #define DWBC_MAX_LAYERS 4
 
+/* Hidden-layer activation of the ActorCritic (rsl_rl get_activation, AC): every layer of the privileged encoder, the four stages of
+ * the history encoder, the actor / critic backbones and the hidden layers of the four heads.  The actor heads' last layer stays tanh,
+ * the critic heads' last layer stays linear.  rsl_rl's "crelu" is a plain ReLU (DWBC_ACT_RELU). */
+enum DwbcActivation {
+  DWBC_ACT_ELU = 0,      /* nn.ELU() (zero: the value of a zero-filled struct) */
+  DWBC_ACT_SELU = 1,     /* nn.SELU() */
+  DWBC_ACT_RELU = 2,     /* nn.ReLU() */
+  DWBC_ACT_LRELU = 3,    /* nn.LeakyReLU(), slope 0.01 */
+  DWBC_ACT_TANH = 4,     /* nn.Tanh() */
+  DWBC_ACT_SIGMOID = 5   /* nn.Sigmoid() */
+};
+
 /* Network shape (AC:86-298).  Parameters live in ONE flat fp32 buffer in
  * ActorCritic.parameters() order (std first); offsets are element offsets into it. */
 typedef struct DwbcNetCfg {
@@ -261,7 +273,7 @@ typedef struct DwbcNetCfg {
    *   2  "3xTF32": every operand is split into the TF32 part the tensor core reads and the exact remainder, three tensor-core
    *      products per GEMM (hi*hi + lo*hi + hi*lo), fp32 accumulation: fp32-grade results on the tensor cores. */
   int32_t precision;
-  int32_t reserved_;
+  int32_t activation;            /* DwbcActivation of the hidden layers; any other value: DWBC_ERR_ARG */
 } DwbcNetCfg;
 
 /* PD torque controller of step() (WG:1262-1295 `_compute_torques`, called `decimation` times per policy step, WG:1175-1183):

@@ -8,7 +8,8 @@ extern "C" {
 #endif
 
 /* One GEMM of the selected implementation (tc: 0 = fp32 CUDA cores, 1 = TF32 tcgen05) on plain row-major device matrices.
- *   mode 0: Y[M,N] = act(X[M,K] W[N,K]^T + b)   mode 1: dX[M,N] = G[M,K] W[K,N]   mode 2: dW[M,N] += G[K,M]^T X[K,N], db += colsum(G) */
+ *   mode 0: Y[M,N] = act(X[M,K] W[N,K]^T + b)   mode 1: dX[M,N] = G[M,K] W[K,N]   mode 2: dW[M,N] += G[K,M]^T X[K,N], db += colsum(G)
+ * act (mode 0): the library's internal activation codes, 0 none, 1 ELU, 2 tanh, 3 SELU, 4 ReLU, 5 leaky ReLU, 6 sigmoid; others DWBC_ERR_ARG */
 int dwbc_debug_gemm(int mode, int tc, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc,
                     const float* bias, float* dbias, int M, int N, int K, int act, dwbc_stream_t stream);
 
